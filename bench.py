@@ -2,7 +2,7 @@
 """bench.py -- Mpixels/s of the portal ray loop on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scene S] [--orbit N]
-                    [--mode owner|p2p|gather] [--format f32|rgba8] [--frontend ron|ir]
+                    [--mode owner|p2p|gather] [--format f32|rgba8] [--frontend ron|ir] [--dump-outputs DIR]
 
 A "step" is one frame of the workload (default: the headline config, portal_in_portal.ron 3840x2160 depth 40, saved
 camera, aa 1): uniform-block upload + ONE launch of the scene's sm_100a ray-loop kernel per GPU.
@@ -185,6 +185,20 @@ def run_reference(args):
 # ------------------------------------------------------------------------------ our arm
 def sha(buf) -> str:
     return hashlib.sha256(memoryview(buf).cast("B")).hexdigest()
+
+
+DUMP_PIXELS = 1 << 20      # --dump-outputs: pixels kept per frame (two frames + their indices: 40 MB of .npy files)
+
+
+def dump_frame(d, name, frame):
+    """--dump-outputs: DIR/<name>.npy = the (h, w, 4) frame's pixels as float32 (n, 4) -- every pixel, or a fixed seeded
+    sample of DUMP_PIXELS of them -- and DIR/pixel_index.npy = their row-major indices (float64)."""
+    import numpy as np
+    n = frame.shape[0] * frame.shape[1]
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(d, f"{name}.npy"), np.ascontiguousarray(frame).reshape(n, 4)[idx].astype(np.float32))
 
 
 def run_ours(args):
@@ -396,6 +410,11 @@ def run_ours(args):
         return {"what": f"{'orbit frame %d' % k if args.orbit else 'last timed frame, saved camera'}, {fmt}, {how}", "sha256": got,
                 "golden": pins.get(key) if pins else None, "match": (got == pins.get(key)) if pins and pins.get(key) else None}
 
+    if args.dump_outputs:
+        frame = assembled_last_frame()          # every rank takes part: owner mode gathers the strips on rank 0
+        if rank == 0:
+            dump_frame(args.dump_outputs, f"frame_{fmt}", frame)
+        del frame
     if not args.orbit:
         rec = hash_value_frame(None)
         if rank == 0:
@@ -456,7 +475,7 @@ def run_ours(args):
             sh.close()
 
     # ---- e2e: the reference-facing call with HOST buffers (RGBA8 frame = get_texture_data), per-frame host work included
-    e2e_steps = min(max(args.steps, 60), 240)      # enough frames that filling and draining the pipeline (one kernel + one copy) is < 2 % of the loop
+    e2e_steps = args.steps          # filling and draining the pipeline (one kernel + one copy) costs about one frame of the loop
     e2e_k = [0]
 
     def e2e_uniforms():
@@ -562,6 +581,8 @@ def run_ours(args):
         barrier()
         hs.close()
     if rank == 0:
+        if args.dump_outputs:
+            dump_frame(args.dump_outputs, "e2e_frame_rgba8", host_bytes)
         pins = golden_pins(args.scene, w, h, depth, args.orbit, e2e_last_k)
         got = sha(np.ascontiguousarray(host_bytes))
         parity["e2e_frame"] = {"what": "last RGBA8 frame delivered to host memory by the e2e loop", "sha256": got,
@@ -668,7 +689,13 @@ def main():
     ap.add_argument("--format", default="f32", choices=["f32", "rgba8"],
                     help="frame format of the timed steps: f32 = float RGBA, 16 B/pixel (the metric's definition, SURVEY.md 8d); "
                          "rgba8 = what the reference's RGBA8 render target holds, 4 B/pixel, quantised by the kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last frame of the timed loop (frame_<format>.npy) and the last host "
+                         "RGBA8 frame of the e2e loop (e2e_frame_rgba8.npy) to DIR as float32 (n, 4) arrays: every pixel, or a "
+                         f"fixed seeded sample of {DUMP_PIXELS} pixels whose row-major indices are in pixel_index.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm renders a sample of the frame in a subprocess; it dumps nothing")
     w, h, d = WORKLOADS[args.scene]
     args.width, args.height, args.depth = args.width or w, args.height or h, args.depth or d
     if args.impl == "reference":

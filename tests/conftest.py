@@ -16,7 +16,8 @@ DEPTH = {"basics": 4, "monoportal": 20, "triple_portal": 40, "portal_in_portal":
 # Oracle and kernel share one pinned numeric profile, transcendentals included (DESIGN.md section 4): every
 # config scene must agree bit for bit.  (exp/log/pow would be the exception; no config scene calls them.)
 BIT_EXACT = ["basics", "monoportal", "triple_portal", "portal_in_portal", "mobius_monoportal"]
-REFERENCE = "/root/reference"
+# The reference's scene files (every scenes/*.ron) and a sample of its scenes/img textures (tools/export_reference_scenes.py)
+REFERENCE_ARCHIVE = os.path.join(GOLDEN, "reference_scenes.tar.xz")
 
 
 def pytest_configure(config):
@@ -51,8 +52,13 @@ def load_tex(name):
 
 
 @pytest.fixture(scope="session")
-def have_reference():
-    return os.path.isdir(REFERENCE)
+def reference(tmp_path_factory):
+    """A directory laid out like the reference checkout: scenes/*.ron and scenes/img/*.png, unpacked from REFERENCE_ARCHIVE."""
+    import tarfile
+    d = tmp_path_factory.mktemp("reference")
+    with tarfile.open(REFERENCE_ARCHIVE) as t:
+        t.extractall(d, filter="data")
+    return str(d)
 
 
 @pytest.fixture(scope="session", autouse=True)

@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import REFERENCE, ROOT
+from conftest import ROOT
 from portal_b200.capi import PortalB200Error
 from portal_b200.host import HostPlayer, HostRenderer, HostScene
 
@@ -254,11 +254,10 @@ def _oracle_probe(orc):
     return probe
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_reference_scene_animations_match_oracle_player():
+def test_reference_scene_animations_match_oracle_player(reference):
     """Every reference scene: its first animations at four times, camera + full uniform table, C++ == oracle."""
     n = 0
-    for path in sorted(glob.glob(f"{REFERENCE}/scenes/*.ron")):
+    for path in sorted(glob.glob(f"{reference}/scenes/*.ron")):
         if os.path.basename(path) == "empty.ron":
             continue
         _, p0, _, hp0 = _pair(path)
@@ -466,15 +465,14 @@ def test_players_agree_on_random_animations(seed, tmp_path):
         _assert_same_state(p, hp, s, hs, (seed, "run", t))
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_per_animation_overrides_of_update_inner_variables():
+def test_per_animation_overrides_of_update_inner_variables(reference):
     """SceneRenderer::update_inner_variables (main.rs:1696-1755), applied right after init_animation_by_name as render-frame
     does: `subspace_degree` becomes Int(500) / Int(1000) for the listed animation names, render depth 100 / fps 600 for others;
     a scene WITHOUT `subspace_degree` leaves the function at the `?` -- before the depth override.  C++ player == oracle
     player, uniform table included."""
     seen = {"degree500": 0, "degree1000": 0, "depth": 0, "fps": 0, "early_exit": 0}
     for scene in ("portal_in_portal", "portal_in_portal_cone", "portal_in_portal_plus_ultra", "teleportation_degrees", "recursive_space"):
-        path = f"{REFERENCE}/scenes/{scene}.ron"
+        path = f"{reference}/scenes/{scene}.ron"
         _, p0, _, _ = _pair(path)
         for an in [a["name"] for a in p0.anim.animations]:
             s, p, hs, hp = _pair(path)

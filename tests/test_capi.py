@@ -40,14 +40,14 @@ def test_library_is_built_for_sm_100a():
 
 @pytest.mark.parametrize("scene", SCENES)
 @pytest.mark.parametrize("persistent", [False, True])
-def test_scene_program_compiles_for_sm_100a(scene, persistent):
+def test_scene_program_compiles_for_sm_100a(scene, persistent, tmp_path):
     r = SceneRenderer(load_ir(scene), device=-1, persistent=persistent)
     src = r.source()
     assert "pe_render_kernel" in src and "__constant__" in src
     assert "!FOR_NUMBER!" not in src
     cubin = r.cubin()
     assert cubin[:4] == b"\x7fELF" and len(cubin) > 10000
-    path = f"/tmp/_pe_test_{scene}_{int(persistent)}.cubin"
+    path = str(tmp_path / f"{scene}_{int(persistent)}.cubin")
     open(path, "wb").write(cubin)
     res = subprocess.run(["cuobjdump", "-res-usage", path], capture_output=True, text=True).stdout
     assert "pe_render_kernel" in res
@@ -209,7 +209,7 @@ def test_bulk_matrix_upload_equals_individual_uploads():
     assert b"no_such_mat" in b._lib.pe_last_error(b._ctx)
 
 
-def test_uniform_block_symbol_and_smem_variant():
+def test_uniform_block_symbol_and_smem_variant(tmp_path):
     """The host finds the uniform block by symbol name after loading the cubin: the name it looks up must be a constant-space
     symbol of exactly the block's size in the cubin -- in the default program (`PE_C`) and in the shared-memory-staging
     variant (`PE_C_UPLOAD`, with `PE_C` a shared image)."""
@@ -218,7 +218,7 @@ def test_uniform_block_symbol_and_smem_variant():
         r = SceneRenderer(ir, device=-1, options=opts)
         size = int(re.search(r"sizeof\(PeConstBlock\) == (\d+)", r.source()).group(1))
         assert len(r.uniform_block(64, 36)) == size
-        path = f"/tmp/_pe_test_symbol_{symbol}.cubin"
+        path = str(tmp_path / f"symbol_{symbol}.cubin")
         open(path, "wb").write(r.cubin())
         ptx_like = subprocess.run(["cuobjdump", "-elf", path], capture_output=True, text=True).stdout
         rows = [ln for ln in ptx_like.splitlines() if re.search(rf"\b{symbol}$", ln.strip())]

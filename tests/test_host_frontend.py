@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import REFERENCE, ROOT, SCENES, load_ir
+from conftest import ROOT, SCENES, load_ir
 from portal_b200 import capi
 from portal_b200.capi import PortalB200Error
 from portal_b200.host import HostRenderer, HostScene
@@ -83,12 +83,11 @@ def test_animation_stages():
         hs.init_stage("nope")
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_every_stage_of_the_config_scenes_matches_oracle_frontend():
+def test_every_stage_of_the_config_scenes_matches_oracle_frontend(reference):
     from oracle import frontend
     n = 0
     for scene in SCENES:
-        path = f"{REFERENCE}/scenes/{scene}.ron"
+        path = f"{reference}/scenes/{scene}.ron"
         for stage in HostScene.from_file(path).stage_names():
             hs = HostScene.from_file(path)
             hs.init_stage(stage)
@@ -101,14 +100,13 @@ def test_every_stage_of_the_config_scenes_matches_oracle_frontend():
 LERP_SCENES = ("half_spheres", "portal_in_portal_cone", "teleportation_degrees", "portal_in_portal_plus_ultra")
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_lerp_matrix_stages_match_oracle_frontend():
+def test_lerp_matrix_stages_match_oracle_frontend(reference):
     """Matrix::Lerp (matrix.rs:614-628) only appears in animation stages of four reference scenes;
     every stage at three times: C++ host == oracle front-end, value for value."""
     from oracle import frontend
     n = 0
     for scene in LERP_SCENES:
-        path = f"{REFERENCE}/scenes/{scene}.ron"
+        path = f"{reference}/scenes/{scene}.ron"
         sc = frontend.load_scene(path)
         hs = HostScene.from_file(path)
         hs.set_formula_camera()
@@ -162,21 +160,19 @@ def test_program_from_host_scene_compiles():
     assert "intersection material `floating_disk`" in src
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("scene", SCENES)
-def test_config_scene_tables_match_oracle_and_golden(scene):
-    hs = HostScene.from_file(f"{REFERENCE}/scenes/{scene}.ron")
+def test_config_scene_tables_match_oracle_and_golden(scene, reference):
+    hs = HostScene.from_file(f"{reference}/scenes/{scene}.ron")
     _assert_same_table(hs.uniform_table(), load_ir(scene))          # committed golden (oracle front-end output)
     if scene in ("triple_portal", "portal_in_portal"):             # use_time scenes: `time` reaches the formulas
         hs.set_time(0.37)
-        _assert_same_table(hs.uniform_table(), _oracle_ir(f"{REFERENCE}/scenes/{scene}.ron", scene, time=0.37))
+        _assert_same_table(hs.uniform_table(), _oracle_ir(f"{reference}/scenes/{scene}.ron", scene, time=0.37))
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_every_reference_scene_loads_and_evaluates():
+def test_every_reference_scene_loads_and_evaluates(reference):
     from oracle import frontend
     n_ok = 0
-    for path in sorted(glob.glob(f"{REFERENCE}/scenes/*.ron")):
+    for path in sorted(glob.glob(f"{reference}/scenes/*.ron")):
         name = os.path.basename(path)[:-4]
         if name == "empty":
             continue
@@ -541,16 +537,11 @@ def test_garbage_formulas_and_mutated_scene_files_are_handled(tmp_path):
     assert loaded + rejected == 400 and rejected > 300
 
 
-def test_vendored_config_scenes_are_the_references_files(have_reference):
+def test_vendored_config_scenes_are_the_references_files(reference):
     """tests/golden/ron/*.ron -- the scene files bench.py and the GPU tests feed to the product's own front-end -- are byte
-    copies of the reference's (checked where the reference checkout exists)."""
-    import glob
-    import pytest
-    if not have_reference:
-        pytest.skip("needs /root/reference")
-    from conftest import REFERENCE, ROOT
+    copies of the reference's."""
     files = sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "ron", "*.ron")))
     assert len(files) == 5
     for f in files:
-        with open(f, "rb") as a, open(os.path.join(REFERENCE, "scenes", os.path.basename(f)), "rb") as b:
+        with open(f, "rb") as a, open(os.path.join(reference, "scenes", os.path.basename(f)), "rb") as b:
             assert a.read() == b.read(), f

@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import DEPTH, GOLDEN, REFERENCE, SCENES, load_ir, load_tex
+from conftest import DEPTH, GOLDEN, SCENES, load_ir, load_tex
 from oracle import formula, frontend, gen_oracle, ron, runner
 
 
@@ -146,10 +146,9 @@ def test_f64_oracle_flags_few_pixels():
     assert bad < 0.01
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("scene", SCENES)
-def test_frontend_regenerates_committed_ir(scene):
-    ir = frontend.scene_ir(frontend.load_scene(f"{REFERENCE}/scenes/{scene}.ron"), scene)
+def test_frontend_regenerates_committed_ir(scene, reference):
+    ir = frontend.scene_ir(frontend.load_scene(f"{reference}/scenes/{scene}.ron"), scene)
     gold = load_ir(scene)
     assert list(ir["uniforms"]) == list(gold["uniforms"])
     for k, u in ir["uniforms"].items():

@@ -9,7 +9,6 @@ frame bound, gives the oracle's pixels bit for bit; an unbound video sampler rea
 import os
 
 import numpy as np
-import pytest
 
 from conftest import ROOT
 from portal_b200.host import HostRenderer, HostScene
@@ -18,7 +17,6 @@ from test_program_on_host import H, W, _bits, _run_on_host
 
 FIXTURE = os.path.join(ROOT, "tests", "fixtures", "video.ron")
 IDENTITY = [1.0, 0, 0, 0, 0, 1.0, 0, 0, 0, 0, 1.0, 0, 0, 0, 0, 1.0]      # eye at the origin looking down +z, like tests/test_analytic.py
-REFERENCE_SCENE = "/root/reference/scenes/boot.dev.ron"
 
 
 def _oracle_scene():
@@ -84,15 +82,15 @@ def test_the_selected_frame_reaches_the_pixels(tmp_path):
     assert (got[H // 2, W // 2, :3] == 0).all() and got[H // 2, W // 2, 3] == 1 and got[:, :, :3].max() > 0
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE_SCENE), reason="reference checkout not present (GPU box)")
-def test_the_references_video_scene_compiles_now():
+def test_the_references_video_scene_compiles_now(reference):
     """`boot.dev` was the one reference scene of 82 the generators rejected (`video1_tex` undefined): both front-ends now give
     it four video samplers, the same uniform table, and the sm_100a generator + NVRTC accept the program."""
     from portal_b200.renderer import SceneRenderer
-    ir = _oracle_ir(REFERENCE_SCENE, "boot.dev")
+    path = os.path.join(reference, "scenes", "boot.dev.ron")
+    ir = _oracle_ir(path, "boot.dev")
     assert [v["name"] for v in ir["videos"]] == ["video1", "video2", "video3", "video4"]
     assert [v["uniform"] for v in ir["videos"]] == [f"video{i}_frame" for i in (1, 2, 3, 4)]
-    hs = HostScene.from_file(REFERENCE_SCENE)
+    hs = HostScene.from_file(path)
     assert [v[0] for v in hs.videos()] == ["video1", "video2", "video3", "video4"]
     _assert_same_table(hs.uniform_table(), ir)
     r = SceneRenderer(ir, device=-1)
